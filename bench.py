@@ -61,7 +61,14 @@ def parse_args():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--job-images", type=int, default=16384, help="images of the configs[4] job, sharded over the N GPUs")
     ap.add_argument("--e2e-chunk", type=int, default=64, help="images per chunk of the host-to-host pipeline")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed decode returned as DIR/<name>.npy "
+                    "(float32 / float64, at most 64 MB; see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs applies to --impl native")
+    return args
 
 
 def measured_peak():
@@ -369,6 +376,44 @@ def parity_check(wl, gen, k_coef, k_oracle, seed):
             "against": "encoder's quantised coefficients (bit-exact gate); oracle samples (gate: max |delta| <= 1)"}
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+DUMP_SAMPLE_BYTES = 32 * 10 ** 6
+DUMP_SEED = 20261020
+
+
+def dump_outputs(out_dir, batch, n):
+    """What the timed decode (jpgpu_batch_decode) returned in its last step, for `n` images of one shape, written so
+    that two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.
+    At most 64 MB in all:
+      status.npy, bytes_read.npy  float64 (n,)      per-image status and scan bytes consumed (jpgpu_batch_results)
+      rgb_sample.npy              float32 (n, K)    K values of every image's decoded (H, W, 3) output, flattened, at
+                                                    positions drawn from a fixed seed (all of them when K = H*W*3)
+      rgb_images.npy              float32 (m, H, W, 3)  the first m images whole, as many as the rest of the 64 MB allows
+    Returns {file name: shape}."""
+    import numpy as np
+    import torch
+    statuses, bytes_read = batch.results()            # synchronises
+    size = int(np.prod(batch.shape(0)))
+    k = min(size, DUMP_SAMPLE_BYTES // (4 * n))
+    rng = np.random.default_rng(DUMP_SEED)
+    pos = np.stack([np.arange(k) if k == size else np.sort(rng.integers(0, size, k)) for _ in range(n)])
+    pos_dev = torch.from_numpy(pos).cuda()
+    sample = torch.empty((n, k), dtype=torch.uint8, device="cuda")
+    for i in range(n):
+        sample[i] = batch.device_tensor(i).reshape(-1).index_select(0, pos_dev[i])
+    arrays = {"status": np.asarray(statuses, np.float64), "bytes_read": np.asarray(bytes_read, np.float64),
+              "rgb_sample": sample.cpu().numpy().astype(np.float32)}
+    room = DUMP_LIMIT_BYTES - sum(a.nbytes for a in arrays.values()) - 1024 * (len(arrays) + 1)   # 1 KB per .npy header
+    m = min(n, room // (4 * size))
+    if m:
+        arrays["rgb_images"] = np.stack([batch.device_tensor(i).cpu().numpy() for i in range(m)]).astype(np.float32)
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {name + ".npy": list(a.shape) for name, a in arrays.items()}
+
+
 def copy_ceiling(in_bytes, out_bytes, reps, barrier, max_over_ranks):
     """Plain pinned cudaMemcpyAsync of the same bytes the end-to-end leg moves (H2D and D2H on two streams at once),
     all ranks together: what the platform's PCIe / host memory system gives at this N, whatever the library does."""
@@ -462,15 +507,18 @@ def main():
     batch.upload_from(wl.buf)
     for _ in range(args.warmup):
         batch.decode()
-    statuses, _ = batch.results()
-    bad = [s for s in statuses if s != 0]
-    if bad:
-        raise SystemExit(f"decode failed for {len(bad)} images, first status {bad[0]}")
     launches0 = batch.launch_count()
     sampler = ClockSampler(local_rank)
     sampler.start()
     time.sleep(0.3)          # let nvidia-smi start sampling before the timed region
     ms_per_step = time_decode(batch, stream, args.steps, barrier, max_over_ranks)
+    # statuses of the last timed step: checked here, not after the warm-up, because with --warmup 0 nothing has been
+    # decoded before the timed region and every image would still read as truncated
+    statuses, _ = batch.results()
+    bad = [s for s in statuses if s != 0]
+    if bad:
+        sampler.stop()
+        raise SystemExit(f"decode failed for {len(bad)} images, first status {bad[0]}")
     per_rank_ms = None
     if world > 1:   # bookkeeping: every rank's own time, so that the line shows how far the slowest is from the rest
         mine = torch.tensor([time_decode.last_local_ms], dtype=torch.float64, device="cuda")
@@ -479,6 +527,9 @@ def main():
         per_rank_ms = [float(t.item()) for t in allms]
     launches = batch.launch_count() - launches0
     value = world * pixels / (ms_per_step * 1e-3) / 1e6
+    dumped = None
+    if args.dump_outputs and rank == 0:   # every rank decodes the same corpus
+        dumped = dump_outputs(args.dump_outputs, batch, n)
     ent_ms, idct_ms, prof = stage_times(batch, stream, args.steps)
     if not sampler.lines:   # very short runs: keep the GPU busy with the same work until the sampler has reported
         t_end = time.perf_counter() + 1.0
@@ -711,7 +762,7 @@ def main():
                        "parallelism": f"images sharded over {world} GPU(s), no collective"},
             "parity": parity, "determinism": determinism, "per_rank_ms_per_step": per_rank_ms,
             "roofline": roofline, "cpu_baseline": cpu, "e2e": e2e, "gpu_launches": launches, "clocks": clocks,
-            "config0_single_image": config0, "extra": extra,
+            "config0_single_image": config0, "extra": extra, "dumped_outputs": dumped,
             "stage_ms": {"entropy": ent_ms, "idct_colour": idct_ms, "note": "stages run one after the other on one stream; "
                          "`value` is timed over jpgpu_batch_decode, which overlaps the image groups of a batch"},
         }
