@@ -96,7 +96,7 @@ constexpr uint32_t kBadEntry = 16u | (16u << 8) | (64u << 16);  // unknown code:
 //   bits 23-29  adv1     | the first symbol alone: what to take when the entry does not hold
 // DC tables have the same format with one symbol per entry, index width kMultiBitsDc, and the code LENGTH in the
 // adv_pre field (the DC difference must be extracted; z = 0 there, so the entry always holds).  0 = no symbol can be
-// determined from the window (code longer than the window, no such code, DC size > 16): single-symbol path.
+// determined from the window (code longer than the window, no such code, DC size >= 16): single-symbol path.
 #ifndef JPGPU_MULTI_BITS
 #define JPGPU_MULTI_BITS 12
 #endif
@@ -305,6 +305,16 @@ JPGPU_HD int32_t extend(uint32_t v, uint32_t top, uint32_t size) {
     return (int32_t)v - (int32_t)(neg & ((1u << size) - 1u));
 }
 
+// The reference's value_correction works in i16, so a DC difference of size category 16 is its 16 raw bits read as
+// an i16, where T.81 EXTEND gives raw - 65535 (first bit 0) or raw (first bit 1).  What to add to extend() for such
+// a symbol; `top` as there.  Only the canonical walk decodes DC category 16 (build_huff_lut, build_multi_lut), so
+// the per-symbol paths never look at it.
+JPGPU_HD int32_t dc16_correction(uint32_t top) { return (top >> 31) ? -65536 : 65535; }
+
+// The reference keeps the DC predictor in f32 and stores it `as i16`, which saturates (decoder.rs:208-210); the
+// predictor itself is not saturated.
+JPGPU_HD int32_t sat_i16(int32_t v) { return v < -32768 ? -32768 : (v > 32767 ? 32767 : v); }
+
 // ------------------------------------------------------------ decoder state
 struct DecCtx {               // per-image constants of the entropy decoder
     const uint32_t* words;    // compacted stream of this image (lane-interleaved)
@@ -435,9 +445,11 @@ JPGPU_HD uint32_t decode_symbol(const DecCtx& cx, DecState& st, int16_t* blk, ui
     const HuffLut* t = z ? st.tac : st.tdc;
     uint32_t e = t->fast[peek >> (32 - kLutBits)];
     if (e & kLinkBit) e = t->pool[(e & 511u) + ((peek << kLutBits) >> (32 - ((e >> 9) & 7u)))];
+    int32_t fix = 0;
     if (e == 0) {
         e = huff_slow(*t, peek);
         if (e == 0) { st.flags |= kStBadCode; e = kBadEntry; }  // huffman.rs:156/162 panic
+        else if ((e & 255u) - ((e >> 8) & 255u) == 16u) fix = dc16_correction(peek << ((e >> 8) & 255u));  // AC sizes are <= 15
     }
     const uint32_t tb = e & 255u, len = (e >> 8) & 255u;
     const int32_t adv = (int32_t)((e >> 16) & 255u);
@@ -449,12 +461,12 @@ JPGPU_HD uint32_t decode_symbol(const DecCtx& cx, DecState& st, int16_t* blk, ui
 #else
         const uint32_t v = size ? top >> (32 - size) : 0u;
 #endif
-        const int32_t val = extend(v, top, size);
+        const int32_t val = extend(v, top, size) + fix;
         if (z == 0) {  // DC difference -> predictor (decoder.rs:208-210)
             if (e & (1u << 24)) st.flags |= kStDcSize;
             int32_t pred;
             if (st.comp == 0) { st.dc0 += val; pred = st.dc0; } else if (st.comp == 1) { st.dc1 += val; pred = st.dc1; } else { st.dc2 += val; pred = st.dc2; }
-            if (WRITE && store_on) blk[buf_index(store_pos[0], swz)] = (int16_t)pred;
+            if (WRITE && store_on) blk[buf_index(store_pos[0], swz)] = (int16_t)sat_i16(pred);
         } else if (WRITE && store_on && val != 0) {  // huffman.rs:183-189: min(run, 64 - len - 1) zeros, then the value
             const int32_t pos = z + adv - 1 < 63 ? z + adv - 1 : 63;
             blk[buf_index(store_pos[pos], swz)] = (int16_t)val;

@@ -133,8 +133,9 @@ int build_huff_lut(const uint8_t bits[16], const uint8_t* vals, int nvals, bool 
     out.maxcode[0] = -1;
     out.maxcode[17] = 0x7fffffff;
     // DC symbols naming a size category > 16 (huffman.rs:202 assert) stay out of both LUT levels: the canonical
-    // walk finds them and reports them, so the per-symbol path never has to look at that flag.
-    if (is_dc) codes.erase(std::remove_if(codes.begin(), codes.end(), [](const Code& c) { return c.val > 16; }), codes.end());
+    // walk finds them and reports them, so the per-symbol path never has to look at that flag.  So does category 16,
+    // whose difference the walk's caller corrects to the reference's i16 value (dc16_correction).
+    if (is_dc) codes.erase(std::remove_if(codes.begin(), codes.end(), [](const Code& c) { return c.val >= 16; }), codes.end());
     // first level: codes of length <= kLutBits fill 2^(kLutBits-len) entries each
     for (const Code& c : codes) {
         if (c.len > kLutBits) continue;
@@ -201,7 +202,7 @@ void build_multi_lut(const uint8_t bits[16], const uint8_t* vals, bool is_dc, st
             if (sym < 0) break;
             uint32_t size, adv;
             bool eob = false;
-            if (is_dc) { if (sym > 16) break; size = (uint32_t)sym; adv = 1; }     // size > 16: huffman.rs:202, single-symbol path reports it
+            if (is_dc) { if (sym >= 16) break; size = (uint32_t)sym; adv = 1; }    // size 16: dc16_correction; > 16: huffman.rs:202 (single-symbol path)
             else if (sym == 0x00) { size = 0; adv = 64; eob = true; }
             else if (sym == 0xf0) { size = 0; adv = 16; }
             else { size = (uint32_t)sym & 15u; adv = ((uint32_t)sym >> 4) + 1u; }

@@ -356,8 +356,10 @@ __device__ __forceinline__ uint32_t lds32v(uint32_t a) { uint32_t v; asm volatil
 __device__ __forceinline__ uint32_t lds8(uint32_t a) { uint32_t v; asm("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
 __device__ __forceinline__ uint2 lds64(uint32_t a) { uint2 v; asm("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(a)); return v; }
 __device__ __forceinline__ void sts32v(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" :: "r"(a), "r"(v) : "memory"); }
-__device__ __forceinline__ void sts16_if(uint32_t a, uint32_t v, bool p) {
-    asm volatile("{\n .reg .pred q;\n setp.ne.u32 q, %2, 0;\n @q st.shared.u16 [%0], %1;\n}" :: "r"(a), "r"(v), "r"((uint32_t)p) : "memory");
+// stores v saturated to [-32768, 32767]
+__device__ __forceinline__ void sts16_sat_if(uint32_t a, int32_t v, bool p) {
+    asm volatile("{\n .reg .pred q;\n .reg .b16 h;\n setp.ne.u32 q, %2, 0;\n cvt.sat.s16.s32 h, %1;\n @q st.shared.u16 [%0], h;\n}"
+                 :: "r"(a), "r"(v), "r"((uint32_t)p) : "memory");
 }
 __device__ __forceinline__ uint32_t smem_addr(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -571,6 +573,9 @@ __device__ __forceinline__ uint32_t fast_long_code(const FastCtx& cx, FastState&
         e = huff_slow(cx.luts[(lut - cx.lut0_addr) / (uint32_t)sizeof(HuffLut)], hi);
         if (e == 0u) { st.flags |= kStBadCode; e = kBadEntry; }
         st.flags |= (e >> 21) & kStDcSize;        // bit 24 -> kStDcSize (8): such DC symbols are only in the canonical tables
+        // DC category 16, also only here: the caller adds fast_extend()'s T.81 value; make it the reference's i16 one
+        const uint32_t len = (e >> 8) & 255u;
+        if ((e & 255u) - len == 16u) st.dcur += dc16_correction(hi << len);   // AC sizes are <= 15
     }
     return e;
 }
@@ -672,8 +677,9 @@ __device__ __forceinline__ uint32_t fast_step(const FastCtx& cx, FastState& st, 
     const uint32_t nz = z + adv;
     if constexpr (WRITE) {
         // huffman.rs:183-189.  Symbols without a value (EOB, ZRL) store a zero at a position the block has not reached.
+        // A DC predictor past the int16 range is stored saturated (sat_i16); AC values (size <= 15) are unchanged by it.
         const uint32_t off = lds8(cx.sp_addr + nz - 1u);   // nz - 1 <= 126: FastTablesT::sp
-        sts16_if(wl.row_swz ^ off, (uint32_t)(is_dc ? st.dcur : val), wl.store_on != 0u);
+        sts16_sat_if(wl.row_swz ^ off, is_dc ? st.dcur : val, wl.store_on != 0u);
     }
     fast_advance(cx, st, st.p + tb);
     if constexpr (WRITE) {
