@@ -991,8 +991,11 @@ constexpr int kRepairJobs = 2 * kInterThreads;
 // One CTA per image. (1) Verification: the chain is right where A(j) == B(j-1).  The broken links
 // (look-back too short for that spot) are collected and each is decoded again from B(j-1) by one
 // thread, segment by segment, until the walk meets the decode recorded for subsequence j — from
-// there on that record was already the true one.  Repeated until the chain holds: the lowest
-// broken link always starts from a correct state, so every iteration extends the correct prefix.
+// there on that record was already the true one.  Repeated until the chain holds.  A round takes
+// the LOWEST kRepairJobs broken links, in ascending order: the lowest broken link starts from a
+// correct state, so it is repaired for good and every round extends the correct prefix by at least
+// one link — nsub - 1 rounds with work at most, whatever the warps' timing.  Links below the lowest
+// one of a round are verified and nothing below it is rewritten, so the next round's sweep starts there.
 // (2) Exclusive prefix scan turning per-subsequence advances into the absolute state at every A
 // (segmented where a restart interval began).
 // MULTI: the repair walks go through the multi-symbol tables like the synchronisation pass (dynamic shared memory:
@@ -1004,7 +1007,7 @@ __global__ void __launch_bounds__(kInterThreads) verify_scan_kernel(BatchDev b) 
     __shared__ FastTables ft;
     __shared__ int32_t s_agg[kInterThreads][5];
     __shared__ RepairJob s_jobs[kRepairJobs];
-    __shared__ uint32_t s_count;
+    __shared__ uint32_t s_warp_broken[kInterThreads / 32];
 
     const uint32_t img = b.img0 + blockIdx.x;
     const uint32_t S = b.sub_bits;
@@ -1014,23 +1017,40 @@ __global__ void __launch_bounds__(kInterThreads) verify_scan_kernel(BatchDev b) 
     const ImgDyn dyn = b.dyn[img];
     const uint32_t nsub = (dyn.stream_bits + S - 1) / S;
     SubInfo* subs = b.subs + im.sub_off;
-    const uint32_t tid = threadIdx.x;
+    const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5;
 
     bool loaded = false;
+    uint32_t from = 1u;   // links below it are verified
 #pragma unroll 1
     for (uint32_t iter = 0; iter <= nsub; iter++) {
-        if (tid == 0) s_count = 0u;
-        __syncthreads();
-        for (uint32_t j = 1 + tid; j < nsub; j += kInterThreads) {
-            const uint32_t start_p = subs[j - 1].pB, start_cz = (subs[j - 1].cz >> 10) & kCzMask;
-            if (start_p != subs[j].pA || start_cz != (subs[j].cz & kCzMask)) {
-                const uint32_t k = atomicAdd(&s_count, 1u);
-                if (k < (uint32_t)kRepairJobs) s_jobs[k] = RepairJob{j, start_p, start_cz};  // the rest waits for the next iteration
+        // the broken links in ascending order, kInterThreads at a time (ballot + per-warp counts), until
+        // kRepairJobs are taken; the rest waits for a later round.  `count` is the same in every thread.
+        uint32_t count = 0u;
+        for (uint32_t base = from; base < nsub && count < (uint32_t)kRepairJobs; base += kInterThreads) {
+            const uint32_t j = base + tid;
+            uint32_t start_p = 0u, start_cz = 0u;
+            bool broken = false;
+            if (j < nsub) {
+                start_p = subs[j - 1].pB;
+                start_cz = (subs[j - 1].cz >> 10) & kCzMask;
+                broken = start_p != subs[j].pA || start_cz != (subs[j].cz & kCzMask);
             }
+            const uint32_t mask = __ballot_sync(0xffffffffu, broken);
+            if (lane == 0u) s_warp_broken[warp] = __popc(mask);
+            __syncthreads();
+            uint32_t k = count + __popc(mask & ((1u << lane) - 1u));
+#pragma unroll
+            for (uint32_t w = 0; w < (uint32_t)(kInterThreads / 32); w++) {
+                const uint32_t c = s_warp_broken[w];
+                if (w < warp) k += c;
+                count += c;
+            }
+            if (broken && k < (uint32_t)kRepairJobs) s_jobs[k] = RepairJob{j, start_p, start_cz};
+            __syncthreads();   // s_warp_broken is rewritten by the next block, s_jobs read below
         }
-        __syncthreads();
-        const uint32_t njobs = min(s_count, (uint32_t)kRepairJobs);
+        const uint32_t njobs = min(count, (uint32_t)kRepairJobs);
         if (njobs == 0u) break;
+        from = s_jobs[0].sub;
         if (!loaded) {
             load_entropy_luts(b, sm, kInterThreads);
             fast_tables_init(ft, sm, threadIdx.x < 32, 32, kInterThreads);

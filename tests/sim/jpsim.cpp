@@ -33,6 +33,8 @@ struct SimBatch {
     // diagnostics
     uint32_t repair_iters = 0;     // most repair iterations any image needed
     uint64_t repairs = 0;          // subsequences decoded again because the look-back had not synchronised
+    uint64_t max_broken = 0;       // most broken links one repair round of one image found
+    uint64_t crowded_rounds = 0;   // repair rounds that found more broken links than one round takes (256)
     uint64_t sync_decodes = 0;     // subsequences decoded by the sync pass
     uint64_t flush_phases = 0, flushed_blocks = 0;
     uint64_t sync_digest = 0;      // hash of the records the synchronisation pass wrote (SubInfo + SegRec)
@@ -142,8 +144,9 @@ void sim_sync(SimBatch& sb, const SeqDesc& sd) {
     }
 }
 
-// mirrors verify_scan_kernel (the order in which the broken links of one iteration are repaired does not matter:
-// every repair starts from a snapshot taken before any of them writes)
+// mirrors verify_scan_kernel: a round takes the lowest 256 broken links (kRepairJobs), the sweep starting at the
+// previous round's lowest one.  Within a round the order of the repairs does not matter: every repair starts from a
+// snapshot of its predecessor taken before any of them writes, and writes only its own subsequence's records.
 void sim_verify_scan(SimBatch& sb, size_t img) {
     std::vector<HuffLut> slots;
     load_slots(sb, img, slots);
@@ -157,15 +160,18 @@ void sim_verify_scan(SimBatch& sb, size_t img) {
     for (int s = 0; s < im.nslots; s++) mslots[s] = sb.plan.mluts.data() + sb.plan.mlut_off[im.slot_lut[s]];
     if (g_sync_multi) cx.mluts = mslots;   // verify_scan_kernel<true>: the repair walks use the multi-symbol tables too
     SubInfo* subs = sb.subs.data() + im.sub_off;
-    uint32_t iters = 0;
+    uint32_t iters = 0, from = 1;
     for (uint32_t iter = 0; iter <= nsub; iter++) {
         std::vector<RepairJob> jobs;
-        for (uint32_t j = 1; j < nsub; j++) {
+        for (uint32_t j = from; j < nsub; j++) {   // all of them, for the diagnostics; the kernel stops at 256
             const uint32_t start_p = subs[j - 1].pB, start_cz = (subs[j - 1].cz >> 10) & kCzMask;
             if (start_p != subs[j].pA || start_cz != (subs[j].cz & kCzMask)) jobs.push_back(RepairJob{j, start_p, start_cz});
         }
+        sb.max_broken = std::max<uint64_t>(sb.max_broken, jobs.size());
+        if (jobs.size() > 256) sb.crowded_rounds++;
         if (jobs.size() > 256) jobs.resize(256);  // kRepairJobs
         if (jobs.empty()) break;
+        from = jobs[0].sub;
         for (const RepairJob& job : jobs) {
             DecState st;
             init_state(cx, st, job.p, (int32_t)(job.cz & 63u), (int32_t)(job.cz >> 6), 0, 0, 0);
@@ -479,7 +485,8 @@ int jpsim_build_multi_lut(const uint8_t bits[16], const uint8_t* vals, int is_dc
 // Runs the whole simulated pipeline on a batch of descriptors.
 //   rgb_out[i]   : W*H*3 bytes (may be NULL)
 //   coef_out[i]  : reference-order coefficients (may be NULL), coef_cap[i] int16 each
-//   diag[4]      : max repair iterations, repaired subsequences, sync-pass subsequences, flush phases
+//   diag[7]      : max repair iterations, repaired subsequences, sync-pass subsequences, flush phases, digest of the
+//                  synchronisation records, most broken links in one repair round, rounds with more than 256 of them
 int jpsim_decode_batch(const jpgpu_image_desc* descs, size_t n, uint8_t* const* rgb_out, int16_t* const* coef_out,
                        const size_t* coef_cap, uint32_t* nblocks /* n x 4 */, int32_t* statuses, uint64_t* bytes_read,
                        uint64_t* diag, uint32_t sub_bits) {
@@ -547,7 +554,10 @@ int jpsim_decode_batch(const jpgpu_image_desc* descs, size_t n, uint8_t* const* 
             for (size_t k = i + 1; k < n && p.frame_part[k] == 2; k++)
                 if (statuses[i] == JPGPU_OK && statuses[k] != JPGPU_OK) statuses[i] = statuses[k];
         }
-    if (diag) { diag[0] = sb.repair_iters; diag[1] = sb.repairs; diag[2] = sb.sync_decodes; diag[3] = sb.flush_phases; diag[4] = sb.sync_digest; }
+    if (diag) {
+        diag[0] = sb.repair_iters; diag[1] = sb.repairs; diag[2] = sb.sync_decodes; diag[3] = sb.flush_phases; diag[4] = sb.sync_digest;
+        diag[5] = sb.max_broken; diag[6] = sb.crowded_rounds;
+    }
     return JPGPU_OK;
 }
 

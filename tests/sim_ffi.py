@@ -101,7 +101,8 @@ def decode_batch(files, layout=_ffi.LAYOUT_SPEC, ext=_ffi.EXT_NONE, sub_bits=0, 
             off += nb[c] * 64
         out.append(r)
     return out, {"repair_iters": diag[0], "repairs": diag[1], "sync_decodes": diag[2], "flush_phases": diag[3],
-                 "sync_digest": diag[4]}
+                 "sync_digest": diag[4], "max_broken": diag[5],
+                 "crowded_rounds": diag[6]}
 
 
 def set_sync_multi(on):
